@@ -5,6 +5,7 @@
     python bench.py --impl reference --gpus N --steps K ...  # CPU arm: the restated reference algorithm (oracle port)
     python bench.py --workload tetra-nerf-original ...       # 256 + 256 samples, uniform sampler (registration.py:20-46)
     python bench.py --mode train ...                         # fused training step (fwd + bwd), BASELINE configs[2] shape
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/<name>.npy
 
 Workload (BASELINE.json configs[1]): 45,000 uniform random points -> scipy Delaunay -> 302,024 tetrahedra,
 4096 camera-like rays per step, `tetra-nerf` config (128 + 128 samples, biased sampler, M = 512), eval-mode
@@ -138,8 +139,17 @@ def mlp_params():
     return p
 
 
+def dump_outputs(directory: str, arrays: dict):
+    """DIR/<name>.npy in float32 (masks as 0/1): the outputs of the last timed step, so that two builds can be compared on them.
+    Each run computes them from the same seeded inputs; training gradients accumulate with atomics, so runs agree on them to rounding."""
+    d = Path(directory)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", torch.as_tensor(a).detach().cpu().float().numpy())
+
+
 def cpu_arm(V, C, field, params, num_rays: int, seed: int, workload: str, nthreads: int = 0):
-    """the restated reference algorithm on the host cores (oracle port); returns (seconds, rays)"""
+    """the restated reference algorithm on the host cores (oracle port); returns (seconds, rays, rendered outputs)"""
     from oracle import oracle as orc
 
     mesh = cpu_arm.mesh if getattr(cpu_arm, "mesh", None) is not None else orc.OracleMesh(V, C)
@@ -148,8 +158,8 @@ def cpu_arm(V, C, field, params, num_rays: int, seed: int, workload: str, nthrea
     w = WORKLOADS[workload]
     cfg = orc.RenderConfig(num_samples=w["num_samples"], num_fine_samples=w["num_fine_samples"], use_biased_sampler=w["use_biased_sampler"])
     t0 = time.perf_counter()
-    orc.render(mesh, torch.from_numpy(field), params, o, d, cfg, nthreads=nthreads)
-    return time.perf_counter() - t0, num_rays
+    img = orc.render(mesh, torch.from_numpy(field), params, o, d, cfg, nthreads=nthreads)
+    return time.perf_counter() - t0, num_rays, img
 
 
 def cpu_threads():
@@ -175,8 +185,10 @@ def run_reference(args, rank, world):
         cpu_arm(V, C, field, params, min(sample, 512), seed=100 + i, workload=args.workload)  # thread pools / allocator warm-up on a short batch
     tot = 0.0
     for i in range(args.steps):
-        dt, _ = cpu_arm(V, C, field, params, sample, seed=200 + i, workload=args.workload)
+        dt, _, img = cpu_arm(V, C, field, params, sample, seed=200 + i, workload=args.workload)
         tot += dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, img)
     value = sample * args.steps / tot
     line = {
         "impl": "reference", "metric": "rays/sec (4096-ray batch, 300k-tet mesh)", "value": value, "unit": "rays/s", "n_gpus": args.gpus,
@@ -242,7 +254,12 @@ def main():
     ap.add_argument("--mlp-precision", default="f16w2", choices=["f16w2", "bf16x3"],
                     help="operand precision of the inference MLP (tn_render_set_mlp_precision): f16w2 = fp16 activations x fp16 hi/lo weights, "
                          "2 MMAs per product, ~2.6e-5 abs on unit-scale density/colour (library default); bf16x3 = 3 MMAs, ~5e-7")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path returned in its last step (rank 0) as DIR/<name>.npy, float32; "
+                         "--mode train adds the loss, the parameter gradients and a fixed sample of 16384 columns of the field gradient")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     if args.rays is None:
         args.rays = 8192 if args.mode == "train" else RAYS_PER_STEP
@@ -351,6 +368,7 @@ def main():
     sampler = ClockSampler(local_rank)
     sampler.start()
     ms_total, _, launches = timed(False)
+    last = {k: v.cpu() for k, v in out.items()} if args.dump_outputs else None  # the timed runs below render into `out` again
     ms_e2e, _, _ = timed(True)
     _, kern_ms, _ = timed(False, profile=True)  # same steps again with CUDA events around every kernel of the library
     # the same timed region with the other operand precision of the MLP (reported beside the headline, never as `value`)
@@ -376,6 +394,8 @@ def main():
         assert torch.equal(mine[:, :3], out["rgb"]) and bool((gathered[:, 3] >= 0).all()), "fused pixel gather: local block differs from the render"
 
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last)
         pk = peaks()
         total_rays = world * R * args.steps
         value = total_rays / (ms_total * 1e-3)
@@ -433,7 +453,7 @@ def main():
                 cpu_arm(V, C, field, params, 256, seed=7 + wi, workload=args.workload)  # warm (thread pools, MKL)
             tot_t, tot_n, k = 0.0, 0, 0
             while tot_t < 10.0 and k < 64:  # ~10 s of CPU work
-                dt, n = cpu_arm(V, C, field, params, 1024, seed=300 + k, workload=args.workload)
+                dt, n, _ = cpu_arm(V, C, field, params, 1024, seed=300 + k, workload=args.workload)
                 tot_t, tot_n, k = tot_t + dt, tot_n + n, k + 1
             line["cpu_baseline"] = {"value": tot_n / tot_t, "unit": "rays/s", "cores": cores, "kind": "port",
                                     "sample": f"{tot_n} rays ({k} batches of 1024) of the same workload through oracle/ "
@@ -481,8 +501,9 @@ def run_train(args, rank, world, dev, V, C, field, params, dist):
     flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
     host_loss = torch.empty((1,), dtype=torch.float32).pin_memory()
 
-    def run(mode_env: str, steps: int, warmup: int, e2e: bool):
+    def run(mode_env: str, steps: int, warmup: int, e2e: bool, capture: bool = False):
         os.environ["TETRANERF_B200_UNFUSED_TRAIN"] = mode_env
+        torch.manual_seed(0)  # the stratified sampler's jitter: the same draws in every run
         model = make_model()
         opt = torch.optim.RAdam(model.parameters(), lr=1e-3)
         tracer = model.get_tetrahedra_tracer()
@@ -498,6 +519,7 @@ def run_train(args, rank, world, dev, V, C, field, params, dist):
             opt.step()
             if e2e:
                 host_loss.copy_(loss.detach().reshape(1), non_blocking=True)
+            return out, loss
 
         for i in range(warmup):
             step(i)
@@ -510,7 +532,7 @@ def run_train(args, rank, world, dev, V, C, field, params, dist):
         for k in range(steps):
             flush.fill_(k & 0xFF)
             ev[k][0].record()
-            step(warmup + k)
+            res = step(warmup + k)
             ev[k][1].record()
         torch.cuda.synchronize(dev)
         launches = tracer.launch_count() - l0
@@ -521,17 +543,24 @@ def run_train(args, rank, world, dev, V, C, field, params, dist):
         t = torch.tensor([ms], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
+        last = None
+        if capture:  # what the caller holds after the last step: outputs, loss, gradients (the field's: a fixed sample of columns)
+            out, loss = res
+            grads = {f"grad.{n}": p.grad for n, p in model.named_parameters() if p.grad is not None and n != "tetrahedra_field"}
+            cols = torch.from_numpy(np.random.default_rng(0).choice(len(V), min(len(V), 16384), replace=False)).to(dev)
+            last = {**out, "rgb_loss": loss, **grads, "grad.tetrahedra_field.sample": model.tetrahedra_field.grad[:, cols]}
+            last = {k: v.detach().cpu() for k, v in last.items()}
         del model, opt
-        return float(t.item()), launches
+        return float(t.item()), launches, last
 
     sampler = ClockSampler(dev.index)
     sampler.start()
-    ms_total, launches = run("0", args.steps, args.warmup, False)
-    ms_e2e, _ = run("0", args.steps, args.warmup, True)
+    ms_total, launches, last = run("0", args.steps, args.warmup, False, capture=bool(args.dump_outputs))
+    ms_e2e, _, _ = run("0", args.steps, args.warmup, True)
     sampler.stop_flag = True
     sampler.join(timeout=2)
     usteps = max(3, args.steps // 4)
-    ms_unfused, _ = run("1", usteps, 3, False)
+    ms_unfused, _, _ = run("1", usteps, 3, False)
     # per-kernel breakdown of one fused step (CUDA events inside the library), plus torch-side pieces timed separately
     os.environ["TETRANERF_B200_UNFUSED_TRAIN"] = "0"
     model = make_model()
@@ -554,6 +583,8 @@ def run_train(args, rank, world, dev, V, C, field, params, dist):
     fr.set_profiling(False)
     del model, opt
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, last)
         pk = peaks()
         total = world * R * args.steps
         S2 = w["num_samples"] + w["num_fine_samples"] + 1

@@ -1,6 +1,5 @@
-"""GPU parity of find_visited_cells / interpolate_values(+backward): vs the CPU oracle (bit-exact) and vs the
-reference's OWN kernels compiled from /root/reference into oracle/_ref (few-ulp, --use_fast_math there)."""
-import ctypes
+"""GPU parity of find_visited_cells / interpolate_values(+backward): vs the CPU oracle (bit-exact) and vs what the
+reference's OWN kernels returned, stored in tests/golden/ref_kernels_golden.npz (few-ulp, --use_fast_math there)."""
 from pathlib import Path
 
 import numpy as np
@@ -12,7 +11,7 @@ from tetranerf.b200 import synthetic as syn
 
 pytestmark = pytest.mark.gpu
 DEV = torch.device("cuda:0")
-REF_SO = Path(__file__).resolve().parents[1] / "oracle" / "_ref" / "libref_kernels.so"
+REF_GOLDEN = Path(__file__).resolve().parent / "golden" / "ref_kernels_golden.npz"
 
 
 @pytest.fixture(scope="module")
@@ -125,46 +124,26 @@ def test_interpolate_autograd_matches_einsum(traced):
     torch.testing.assert_close(field.grad, f2.grad, rtol=1e-4, atol=1e-4)
 
 
-@pytest.mark.skipif(not REF_SO.exists(), reason="oracle/_ref not built (needs /root/reference at build time)")
 def test_against_reference_kernels(traced):
-    """oracle/_ref/libref_kernels.so = src/tetrahedra_tracer.cu of the reference, compiled unmodified for
-    sm_100a with the reference's flags (-O3 --use_fast_math).  Indices exact; floats within a few ulp."""
+    """The reference's src/tetrahedra_tracer.cu, compiled unmodified for sm_100a with the reference's flags (-O3 --use_fast_math),
+    on inputs of the `traced` problem: its outputs are stored with those inputs in tests/golden/ref_kernels_golden.npz
+    (tests/golden/make_ref_kernels_golden.py).  Indices exact; floats within a few ulp."""
     from tetranerf import cpp
 
-    ref = ctypes.CDLL(str(REF_SO))
-    tr, out, dist, V, C = traced
-    srt = torch.sort(dist, dim=1).values.contiguous()
-    R, S = srt.shape
-    M = out["visited_cells"].shape[1]
-    g = tr.find_visited_cells(out["num_visited_cells"], out["visited_cells"], out["barycentric_coordinates"], out["hit_distances"],
-                              out["vertex_indices"], srt)
-    mask = torch.zeros((R, S), dtype=torch.bool, device=DEV)
-    cell = torch.full((R, S), -1, dtype=torch.int32, device=DEV)
-    bary = torch.zeros((R, S, 3), dtype=torch.float32, device=DEV)
-    verts = torch.full((R, S, 4), -1, dtype=torch.int32, device=DEV)
-    p = lambda t: ctypes.c_void_p(t.data_ptr())
-    torch.cuda.synchronize()
-    rc = ref.ref_find_matched_cells(ctypes.c_size_t(R), ctypes.c_size_t(S), ctypes.c_size_t(M), p(torch.from_numpy(C).to(DEV)),
-                                    p(out["num_visited_cells"]), p(out["visited_cells"]), p(out["hit_distances"]),
-                                    p(out["barycentric_coordinates"]), p(srt), p(out["vertex_indices"]), p(cell), p(verts), p(mask), p(bary))
-    assert rc == 0
-    assert torch.equal(mask, g["mask"]) and torch.equal(cell, g["cell_indices"]) and torch.equal(verts, g["vertex_indices"])
-    torch.testing.assert_close(bary, g["barycentric_coordinates"], rtol=2e-6, atol=2e-6)
+    gold = dict(np.load(REF_GOLDEN))
+    t = lambda k: torch.from_numpy(gold[k]).to(DEV)
+    tr = traced[0]  # holds the mesh the stored hit lists were traced on
+    g = tr.find_visited_cells(t("num_visited_cells"), t("visited_cells"), t("barycentric_coordinates"), t("hit_distances"),
+                              t("vertex_indices"), t("distances"))
+    assert torch.equal(t("ref_mask"), g["mask"]) and torch.equal(t("ref_cell_indices"), g["cell_indices"])
+    assert torch.equal(t("ref_vertex_indices"), g["vertex_indices"])
+    torch.testing.assert_close(t("ref_barycentric_coordinates"), g["barycentric_coordinates"], rtol=2e-6, atol=2e-6)
     # interpolation forward: FFMA chain -> expect bit-exact; backward: atomics -> tolerance
-    field = torch.from_numpy(syn.random_field(len(V), 64)).to(DEV)
-    N = R * S
-    res = torch.empty((64, N), dtype=torch.float32, device=DEV)
-    rc = ref.ref_interpolate_values4(ctypes.c_uint32(len(V)), ctypes.c_uint32(N), ctypes.c_uint32(64), p(g["vertex_indices"]),
-                                     p(g["barycentric_coordinates"]), p(field), p(res))
-    assert rc == 0
-    mine = cpp.interpolate_values(g["vertex_indices"], g["barycentric_coordinates"], field)
-    torch.testing.assert_close(mine.reshape(N, 64), res.T.contiguous(), rtol=1e-6, atol=1e-6)
-    frac_exact = (mine.reshape(N, 64) == res.T).float().mean().item()
+    vi, bc, field = t("interp_vertex_indices"), t("interp_barycentric_coordinates"), t("field")
+    res = t("ref_interpolated")
+    mine = cpp.interpolate_values(vi, bc, field)
+    torch.testing.assert_close(mine, res, rtol=1e-6, atol=1e-6)
+    frac_exact = (mine == res).float().mean().item()
     assert frac_exact > 0.99, frac_exact
-    gin = torch.randn((N, 64), device=DEV)
-    gref = torch.zeros((64, len(V)), device=DEV)
-    rc = ref.ref_interpolate_values_backward4(ctypes.c_uint32(len(V)), ctypes.c_uint32(N), ctypes.c_uint32(64), p(g["vertex_indices"]),
-                                              p(g["barycentric_coordinates"]), p(gin.T.contiguous()), p(gref))
-    assert rc == 0
-    gmine = cpp.interpolate_values_backward(g["vertex_indices"], g["barycentric_coordinates"], field, gin)
-    torch.testing.assert_close(gmine, gref, rtol=1e-4, atol=1e-4)
+    gmine = cpp.interpolate_values_backward(vi, bc, field, t("grad_interpolated"))
+    torch.testing.assert_close(gmine, t("ref_field_grad"), rtol=1e-4, atol=1e-4)
